@@ -376,6 +376,18 @@ def run_native(args):
     eng = Engine(graph, B, emb, mode=mode, device=str(dev), world_size=world, use_cuda_graph=not args.no_graph,
                  comm=args.comm, cls_weight=wl['cls_weight'], num_classes=ncls)
     eng.set_lr(0.1)
+    restore_initial_state = None
+    if args.dump_outputs:
+        # Training from the random initialisation is chaotic: the ordering differences of atomically accumulated sums
+        # (~1e-7) grow ~100x per step, so after a few steps two runs of the same build differ by ~1e-2.  The dumped
+        # step therefore starts from the seeded initial state (a ~15 MB device copy inside the timed window), which makes
+        # its outputs a function of the arguments alone.
+        state = (eng.P, eng.V, eng.S, eng.lr_dev)
+        initial = [t.clone() for t in state]
+
+        def restore_initial_state():
+            for t, t0 in zip(state, initial):
+                t.copy_(t0)
 
     # synthetic data: N(0,1) images, seed 1000+rank (SURVEY.md section 8d); a small pool cycled through
     gen = torch.Generator().manual_seed(1000 + rank)
@@ -391,13 +403,15 @@ def run_native(args):
             dist.barrier()
             torch.cuda.synchronize(dev)
 
-    def timed(loader, steps, read_loss):
+    def timed(loader, steps, read_loss, before_last=None):
         barrier()
         t0 = torch.cuda.Event(enable_timing=True)
         t1 = torch.cuda.Event(enable_timing=True)
         t0.record()
         last, pending = None, None
         for s in range(steps):
+            if s == steps - 1 and before_last is not None:
+                before_last()
             loader(s)
             eng.train_step()
             if read_loss:
@@ -429,7 +443,9 @@ def run_native(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_res, _ = timed(resident, args.steps, False)
+    ms_res, _ = timed(resident, args.steps, False, restore_initial_state)
+    # the headline path's last step, read before the end-to-end pass trains on
+    outputs = step_outputs(eng) if (args.dump_outputs and rank == 0) else None
     ms_e2e, last_loss = timed(from_host, args.steps, True)
     clocks = sampler.stop() if rank == 0 else None
 
@@ -501,8 +517,38 @@ def run_native(args):
             'retrieval': retrieval, 'cpu_baseline': cpu, 'clocks': clocks, 'peaks': pk,
         }
         print(json.dumps(line))
+    if outputs is not None:
+        dump_outputs(outputs, args.dump_outputs)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_MAX_ELEMENTS = 4 << 20          # per array; a larger one is written as a fixed, seeded sample of this many elements
+
+
+def step_outputs(eng):
+    """What a caller of Engine.train_step receives after the step: per-sample loss / accuracy (and classifier loss /
+    accuracy), the embeddings (and class probabilities), gradient norm and L2 term, and the updated weights (BatchNorm
+    moving statistics included) and momentum buffers, each concatenated in weight-name order."""
+    out = {k: np.asarray(v, np.float32) for k, v in eng.per_sample_metrics().items()}
+    out['embeddings'] = eng.act[eng.head_node.output.name].cpu().numpy()
+    if eng.xent_node is not None:
+        out['class_probabilities'] = eng.act[eng.xent_node.output.name].cpu().numpy()
+    out['grad_norm_and_l2'] = np.array(eng.grad_norm_and_reg(), np.float64)
+    for name, d in (('weights', eng.get_weights()), ('velocity', eng.get_velocity())):
+        out[name] = np.concatenate([d[k].ravel() for k in sorted(d)])
+    return out
+
+
+def dump_outputs(outputs, out_dir):
+    """DIR/<name>.npy per array; arrays above DUMP_MAX_ELEMENTS are flattened and sampled at indices that depend only on
+    their length, so that two builds given the same arguments write comparable files."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        if a.size > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.RandomState(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))
+            a = a.ravel()[idx]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def eng_bytes(eng):
@@ -533,7 +579,12 @@ def main():
     ap.add_argument('--skip-retrieval', action='store_true')
     ap.add_argument('--skip-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed training step computed as DIR/<name>.npy (float32 / float64); that '
+                         'step starts from the seeded initial weights, so the files depend on the arguments alone')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3)
     if args.impl == 'reference':
         run_reference(args)

@@ -410,3 +410,17 @@ def test_tensor_core_coverage_of_the_baseline_networks(built_lib):
     s2 = [v for v in wrn.values() if v[0] == 3 and v[1] == 2]
     assert len(s2) == 2 and all(v[3:] == (0, 1, 1) for v in s2)
     assert [n for n, v in wrn.items() if v[3:] == (0, 0, 0)] == [next(iter(wrn))]     # only the 3-channel stem
+
+
+def test_bench_dump_outputs_samples_large_arrays_reproducibly(tmp_path):
+    """bench.py --dump-outputs: arrays up to DUMP_MAX_ELEMENTS are written whole; a larger one as a sample at indices
+    that depend only on its length, so that two runs (or two builds) write the same elements."""
+    import bench
+    n = bench.DUMP_MAX_ELEMENTS
+    outs = {'small': np.arange(6, dtype=np.float64).reshape(2, 3), 'big': np.arange(n + 1000, dtype=np.float32)}
+    for run in ('a', 'b'):
+        bench.dump_outputs(outs, str(tmp_path / run))
+    np.testing.assert_array_equal(np.load(str(tmp_path / 'a' / 'small.npy')), outs['small'])
+    a, b = (np.load(str(tmp_path / run / 'big.npy')) for run in ('a', 'b'))
+    assert a.dtype == np.float32 and a.shape == (n,) and np.array_equal(a, b)
+    assert (np.diff(a) > 0).all() and a[-1] < n + 1000           # distinct elements, in index order

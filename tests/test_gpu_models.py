@@ -691,3 +691,38 @@ def test_cli_finetune_from_dump(tmp_path, capsys):
     # after the full-model epoch every backbone tensor has moved away from the dump
     name = [n for n in pre if n.endswith('/kernel') and n != 'embedding/kernel'][0]
     assert pre[name].shape == snap['weights'][name].shape and not np.array_equal(pre[name], snap['weights'][name])
+
+
+def test_bench_dump_outputs_are_the_last_timed_step_and_reproducible(tmp_path):
+    """bench.py --dump-outputs: the last timed training step's per-sample loss / accuracy, embeddings, gradient norm and
+    updated weights / momentum as float32 / float64 .npy files.  That step starts from the seeded initial state, so two
+    runs whose last step trains on the same batch of the 4-batch pool (--steps 2 and --steps 6) write the same numbers up
+    to the ordering of atomically accumulated sums (measured on the B200: ~1e-7 in the forward pass, up to 3e-3 of the
+    largest momentum value)."""
+    import subprocess
+    import sys
+    from semantic_embeddings_b200 import utils
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for steps in (2, 6):
+        d = tmp_path / ('steps%d' % steps)
+        out = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--steps', str(steps), '--warmup', '3',
+                              '--skip-retrieval', '--skip-cpu-baseline', '--dump-outputs', str(d)],
+                             capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])['steps'] == steps
+        dumps.append({f[:-4]: np.load(str(d / f)) for f in sorted(os.listdir(str(d)))})
+    a, b = dumps
+    assert sorted(a) == ['acc', 'embeddings', 'grad_norm_and_l2', 'loss', 'velocity', 'weights']
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert a['loss'].shape == (128,) and a['embeddings'].shape == (128, 100) and a['grad_norm_and_l2'].dtype == np.float64
+    np.testing.assert_allclose(np.linalg.norm(a['embeddings'], axis=1), 1.0, atol=1e-5)
+    g = utils.build_network(100, 'resnet-110-fc', input_channels=3)
+    assert a['weights'].size == sum(int(np.prod(p.shape)) for p in g.params.values())
+    assert np.isfinite(a['weights']).all() and np.abs(a['velocity']).max() > 0
+    tol = {'velocity': 3e-2, 'grad_norm_and_l2': 1e-3}
+    for k in a:
+        err = rel_max(b[k], a[k])
+        report('bench_dump_outputs', array=k, rel_max_err=err)
+        assert err <= tol.get(k, 1e-4), (k, err)
